@@ -13,6 +13,7 @@ A STEP = one pass over SUB x 297 = 4752 frames (16 batches; the same 297 images 
 keyframes fall on a differently oriented copy of the room).  With the driver's --steps 20 the timed region is > 1 s.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--nfeatures 2000] [--no-cpu]
+                  [--dump-outputs DIR]
 
 N > 1 (torchrun, one rank per GPU): STRONG scaling -- the 4752 frames of a step are sharded in contiguous ranges
 (+1 halo frame each, re-extracted locally), every rank maps its own keyframes, and ocm_merge_nccl (the only collective
@@ -296,6 +297,47 @@ except Exception:
 EXPERIMENTAL_STAGE_BITS = {"orient_desc": 1}
 
 
+DUMP_FRAMES = 48       # frames of the last batch whose keypoints / descriptors / matches --dump-outputs writes
+DUMP_MAX_LEAVES = 1 << 20
+
+
+def _device_array(torch, ptr: int, nbytes: int):
+    """Host copy of nbytes of device memory at ptr, as uint8."""
+    class _View:
+        __cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (ptr, False), "version": 3}
+    return torch.as_tensor(_View(), device="cuda").cpu().numpy()
+
+
+def dump_outputs(out_dir, torch, trk, nframes, pcm):
+    """What a caller of the timed path receives after its last step, as float32 .npy files (< 64 MB in all): per frame
+    of the last batch its keypoint and match counts; for a fixed, seeded sample of DUMP_FRAMES of those frames its
+    keypoints (x, y, size, angle, response, octave, class_id), descriptors (one value per byte) and cur->last match
+    vector, zero / -1 past the frame's keypoint count; and the occupancy map's leaves sorted by key (key x, y, z,
+    log-odds, r, g, b), a seeded sample of DUMP_MAX_LEAVES of them if there are more."""
+    from orb_slam2_ssd_semantic_b200.extractor import KP_DTYPE
+    os.makedirs(out_dir, exist_ok=True)
+    (p_kps, p_desc, p_nkp, p_c2l, p_nm), cap = trk.device_results()
+    nkp = _device_array(torch, p_nkp, 4 * nframes).view(np.int32)
+    nm = _device_array(torch, p_nm, 4 * nframes).view(np.int32)
+    frames = np.sort(np.random.default_rng(0).choice(nframes, min(DUMP_FRAMES, nframes), replace=False))
+    kps = _device_array(torch, p_kps, KP_DTYPE.itemsize * cap * nframes).view(KP_DTYPE).reshape(nframes, cap)[frames]
+    desc = _device_array(torch, p_desc, 32 * cap * nframes).reshape(nframes, cap, 32)[frames]
+    c2l = _device_array(torch, p_c2l, 4 * cap * nframes).view(np.int32).reshape(nframes, cap)[frames]
+    valid = np.arange(cap)[None, :] < nkp[frames][:, None]
+    kp = np.stack([kps[f].astype(np.float32) for f in KP_DTYPE.names], -1)
+    keys, logodds, rgb = pcm.export_leaves()
+    order = np.argsort(keys[:, 0].astype(np.uint64) | (keys[:, 1].astype(np.uint64) << np.uint64(16)) |
+                       (keys[:, 2].astype(np.uint64) << np.uint64(32)), kind="stable")
+    if len(order) > DUMP_MAX_LEAVES:
+        order = order[np.sort(np.random.default_rng(0).choice(len(order), DUMP_MAX_LEAVES, replace=False))]
+    arrays = {"nkp": nkp, "nmatch": nm, "sample_frames": frames,
+              "keypoints": np.where(valid[..., None], kp, 0), "descriptors": np.where(valid[..., None], desc, 0),
+              "cur2last": np.where(valid, c2l, -1),
+              "map_leaves": np.concatenate([keys[order], logodds[order, None], rgb[order]], 1)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float32))
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -386,6 +428,9 @@ def run_b200(args):
     st.sync(); st_b.sync(); pcm.sync()
     barrier()
     clocks = sampler.result()
+    if args.dump_outputs and rank == 0:
+        # every batch of a step tracks the same frames; the last one ran on the handle its index selects in step_device
+        dump_outputs(args.dump_outputs, torch, st if (len(plan) - 1) % 2 == 0 else st_b, plan[-1]["n"], pcm)
     ms_total, map_ms = e0.elapsed_time(e1), em0.elapsed_time(em1)
     launches = st.launch_count() + st_b.launch_count() + pcm.launch_count() - launches0
     # per-stage durations for the roofline: ONE more step, serial on one handle with the stage events on (inside the
@@ -483,7 +528,7 @@ def run_b200(args):
     run_host(1)
     barrier()
     t0 = time.perf_counter()
-    e2e_steps = max(2, min(args.steps, 16))   # 16 steps x ~82 ms: the e2e timed region exceeds 1 s at the default --steps 20
+    e2e_steps = args.steps
     which, nlast = run_host(e2e_steps)
     torch.cuda.synchronize()
     t_e2e = time.perf_counter() - t0
@@ -622,6 +667,7 @@ def main():
     ap.add_argument("--nfeatures", type=int, default=2000, help="ORBextractor nfeatures (configs[2]: 2000; TUM yaml: 1000)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":

@@ -396,7 +396,7 @@ _reflib = None
 
 
 def refsrc_available() -> bool:
-    return os.path.exists(_REFSO) or os.path.exists("/root/reference/src/ORBextractor.cc")
+    return os.path.exists(_REFSO)
 
 
 def reflib() -> C.CDLL:
@@ -935,7 +935,7 @@ _perflib = None
 
 
 def refperfect_available() -> bool:
-    return os.path.exists(_PERFSO) or os.path.exists("/root/reference/perfect/src/Frame.cc")
+    return os.path.exists(_PERFSO)
 
 
 def perfect_frames(gray: np.ndarray, depth: np.ndarray, mask: np.ndarray, nfeatures=1000, scale=1.2, nlevels=8, ini_th=20,

@@ -82,11 +82,12 @@ def test_filter_keypoints_rule():
 def test_filter_oracle_equals_the_reference_masked_constructor():
     """oracle == the `perfect` tree's OWN code: perfect/src/Frame.cc compiled unmodified (oracle/_ref/librefperfect.so).
     filter_keypoints(mask, what the plain RGB-D constructor keeps) must be what the masked constructor keeps (:328-427),
-    bit for bit -- with a real dynamic mask (filter on), with a mask at 64.6 % (filter off, :358) and with stray values."""
+    bit for bit -- with a real dynamic mask (filter on), with a mask at 64.6 % (filter off, :358) and with stray values.
+    The reference's outputs are recorded (tests/reference_outputs.py); live where the library exists."""
     from oracle import ref
-    if not ref.refperfect_available():
-        pytest.skip("neither oracle/_ref/librefperfect.so nor the reference is on this box")
     from orb_slam2_ssd_semantic_b200 import synth
+    from tests.reference_outputs import Reference
+    R = Reference("test_filter_oracle_equals_the_reference_masked_constructor", ref.refperfect_available())
     ws = synth.WallStream(seed=1234, n=2)
     gray, depth, _, _ = ws.frame(1)
     real = O.mask_from_flow(synth.flow_field(11, 240, 320), 40.0)
@@ -96,15 +97,16 @@ def test_filter_oracle_equals_the_reference_masked_constructor():
     stray = np.ones((480, 640), np.uint8)
     stray[:, 200:330] = 2                                  # "val == 1" only: a 2 is outside
     stray[100:140] = 0
+    # what the plain constructor keeps is the extractor's output (zero distortion), which tests/test_refsrc_cpu.py pins
+    kp, dp = ref.RefExtractor(1000, 1.2, 8, 20, 7)(gray)
+    assert len(kp) > 900
     for name, mask in (("real", real), ("off", off), ("stray", stray)):
-        (kp, dp), (km, dmk) = ref.perfect_frames(gray, depth, mask)
-        assert len(kp) > 900
         ko, do = O.filter_keypoints(mask, kp, dp)
-        assert len(ko) == len(km) and ko.tobytes() == km.tobytes() and (do == dmk).all(), name
+        R.same(name, ((kp, dp), (ko, do)), lambda: ref.perfect_frames(gray, depth, mask))
         if name == "off":
-            assert len(km) == len(kp)
+            assert len(ko) == len(kp)
         else:
-            assert 0 < len(km) < len(kp)
+            assert 0 < len(ko) < len(kp)
 
 
 @pytest.mark.parametrize("rows,cols,gray_shape,thr,seed", [(2, 2, (4, 4), 40.0, 1), (2, 9, (5, 19), 40.0, 2), (31, 17, (63, 34), 55.5, 3),
